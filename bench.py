@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- ZigMa denoiser hot path on B200 (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config NAME]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config NAME] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 A "step" is one denoiser evaluation (ZigMa.forward at the per-GPU batch of the workload, bf16, synthetic weights /
@@ -404,9 +404,10 @@ def other_kernel_rooflines(name, bs, dev):
     return out
 
 
-def run_workload(name, bs, K, W, dev, world, rank, use_graph=True, with_e2e=True):
+def run_workload(name, bs, K, W, dev, world, rank, use_graph=True, with_e2e=True, keep_outputs=False):
     """Builds the model of workload `name`, times K Euler steps (one CUDA graph for the whole K-step loop), the end-to-end
-    leg with host buffers, and returns the measurements.  Every rank calls this; collectives only when world > 1."""
+    leg with host buffers, and returns the measurements (with keep_outputs, also the final latents of the timed loop under
+    "outputs").  Every rank calls this; collectives only when world > 1."""
     import torch
     import torch.distributed as dist
     from zigma_b200 import ZigMa, _lib, synth
@@ -463,6 +464,7 @@ def run_workload(name, bs, K, W, dev, world, rank, use_graph=True, with_e2e=True
         e1.record()
         barrier()
         torch.cuda.profiler.stop()
+        outputs = {"latents": full.float().cpu().numpy()} if keep_outputs else None
         ms = e0.elapsed_time(e1)
         clk = clocks.stop() if rank == 0 else None
         if world > 1:
@@ -471,7 +473,7 @@ def run_workload(name, bs, K, W, dev, world, rank, use_graph=True, with_e2e=True
             ms = tm.item()
         assert torch.isfinite(full.float()).all()
         res = {"ms": ms, "ms_per_step": ms / K, "per_eval": per_eval, "clocks": clk, "bs": bs, "warm_steps": n_warm * K,
-               "tokens_per_s": bs * world * wl["tokens"] * K / (ms * 1e-3)}
+               "tokens_per_s": bs * world * wl["tokens"] * K / (ms * 1e-3), "outputs": outputs}
 
         if with_e2e:
             # ---- e2e: public API with HOST buffers: pinned latents/t H2D, forward, result D2H, every step
@@ -508,6 +510,23 @@ def run_workload(name, bs, K, W, dev, world, rank, use_graph=True, with_e2e=True
     return res
 
 
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, arrays):
+    """Writes each array as <out_dir>/<name>.npy in float32, so that two builds run with the same arguments can be compared
+    output for output.  An array larger than DUMP_LIMIT_BYTES is replaced by a fixed, seeded sample of its leading-dimension
+    rows (sorted; the same rows for the same shape in every run)."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        a = np.ascontiguousarray(a, dtype=np.float32)
+        if a.nbytes > DUMP_LIMIT_BYTES:
+            rows = np.random.default_rng(0).choice(a.shape[0], DUMP_LIMIT_BYTES // (a.nbytes // a.shape[0]), replace=False)
+            a = a[np.sort(rows)]
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -521,7 +540,11 @@ def main():
     ap.add_argument("--no-graph", action="store_true", help="launch kernels eagerly (for ncu launch lists)")
     ap.add_argument("--no-train", action="store_true", help="skip the forward+backward (training step) side measurement")
     ap.add_argument("--no-configs", action="store_true", help="skip the side measurements of the other BASELINE configs")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the final latents of the timed sampling loop to DIR/latents.npy "
+                    "(float32; inputs and weights are seeded, so runs with the same arguments can be compared)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local = int(os.environ.get("LOCAL_RANK", "0"))
@@ -542,7 +565,9 @@ def main():
     wl = WORKLOADS[name]
     bs = args.bs or wl["bs"]
 
-    main_res = run_workload(name, bs, K, W, dev, world, rank, use_graph=not args.no_graph)
+    main_res = run_workload(name, bs, K, W, dev, world, rank, use_graph=not args.no_graph, keep_outputs=bool(args.dump_outputs))
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, main_res.pop("outputs"))
     roof = scan_roofline(name, bs, dev, main_res["ms_per_step"], wl["cfg"]["depth"]) if rank == 0 else None
     if world > 1:
         dist.barrier()

@@ -1,116 +1,63 @@
 """CPU: the binding INTEGRATION.md documents for a reference maintainer (section 1: register ctypes-backed stand-ins for the
 two native extension modules before the reference is imported) is EXECUTED here -- the shim text is taken verbatim from the
-document, the reference's own interface files are loaded on top of it, and the reference's autograd Functions run forward and
-backward through it.  The CUDA-only raw ops the shim calls are replaced by CPU fakes built on the oracle, so what is verified
+document, and the calls the reference's own autograd Functions make into the two modules (selective_scan_fn forward and
+backward, causal_conv1d_fn forward and backward, recorded from the unmodified reference by oracle/gen_golden_shim.py) are
+replayed against it.  The CUDA-only raw ops the shim calls are replaced by CPU fakes built on the oracle, so what is verified
 is the glue: module / function names, argument order, the layout of the returned lists, the state handed from fwd to bwd."""
-import importlib.util
-import os
-import re
+import json
 import sys
 
-import pytest
 import torch
 
-from oracle import zigma_oracle as zo
-from util import ROOT
-
-REF = "/root/reference"
-pytestmark = pytest.mark.skipif(not os.path.isdir(os.path.join(REF, "dis_mamba")), reason="needs the reference tree (build container only)")
+from oracle import gen_golden_shim as gs
+from util import gold
 
 
-def _load(name, path):
-    spec = importlib.util.spec_from_file_location(name, path, submodule_search_locations=[os.path.dirname(path)] if path.endswith("__init__.py") else None)
-    mod = importlib.util.module_from_spec(spec)
-    sys.modules[name] = mod
-    spec.loader.exec_module(mod)
-    return mod
+def _replay(g):
+    """Each recorded call on the registered module; an argument recorded as an element of an earlier result is that element."""
+    results = []
+    for call in json.loads(bytes(g["trace_json"]).decode()):
+        args = []
+        for kind, *ref in call["args"]:
+            if kind == "arr":
+                args.append(torch.from_numpy(g[ref[0]]))
+            elif kind == "ret":
+                args.append(results[ref[0]][ref[1]])
+            else:
+                args.append(ref[0])
+        res = getattr(sys.modules[call["module"]], call["fn"])(*args)
+        results.append(list(res) if isinstance(res, (list, tuple)) else [res])
+    return results
 
 
 def test_integration_md_shim_runs_under_the_reference_interfaces(monkeypatch):
-    text = open(os.path.join(ROOT, "INTEGRATION.md")).read()
-    blocks = re.findall(r"```python\n(.*?)```", text, flags=re.S)
-    shim = next(b for b in blocks if "zigma_shims.py" in b)
-
-    import zigma_b200.selective_scan_interface as zsi
-    import zigma_b200.causal_conv1d_interface as zci
-    calls = []
-
-    def fake_scan_fwd(u, delta, A, B, C, D=None, z=None, delta_bias=None, delta_softplus=False, z_rowmap=None,
-                      want_last_state=True, want_ckpt=False, out=None, dt_proj=None):
-        calls.append("scan_fwd")
-        o, last = zo.selective_scan(u, delta, A, B[:, 0] if B.dim() == 4 else B, C[:, 0] if C.dim() == 4 else C, D, z, delta_bias,
-                                    delta_softplus, return_last_state=True)
-        return o, (last if want_last_state else None), ("CKPT" if want_ckpt else None), (u, delta, z, B, C, D, delta_bias, A)
-
-    def fake_scan_bwd(saved, ckpt, dout, delta_softplus, dz_out=None, z_rowmap=None):
-        calls.append("scan_bwd")
-        assert ckpt == "CKPT", "the checkpoint object of the forward must reach the backward"
-        u, delta, z, B, C, D, delta_bias, A = saved
-        leaves = [t.detach().clone().requires_grad_() if t is not None else None for t in (u, delta, A, B, C, D, delta_bias, z)]
-        lu, ld, lA, lB, lC, lD, lb, lz = leaves
-        with torch.enable_grad():      # (we are inside the reference Function's backward: grad mode is off)
-            o = zo.selective_scan(lu, ld, lA, lB[:, 0], lC[:, 0], lD, lz, lb, delta_softplus)
-        o.backward(dout)
-        g = lambda t: None if t is None else t.grad
-        return g(lu), g(ld), g(lA), g(lB), g(lC), g(lD), g(lb), g(lz)
-
-    def fake_conv_fwd(x, w, b, silu, x_rowmap=None, out=None):
-        calls.append("conv_fwd")
-        return zo.causal_conv1d(x, w, b, "silu" if silu else None)
-
-    def fake_conv_bwd(x, w, b, dout, silu, dx_out=None, x_rowmap=None):
-        calls.append("conv_bwd")
-        lx, lw = x.detach().clone().requires_grad_(), w.detach().clone().requires_grad_()
-        lb = None if b is None else b.detach().clone().requires_grad_()
-        with torch.enable_grad():
-            yy = zo.causal_conv1d(lx, lw, lb, "silu" if silu else None)
-        yy.backward(dout)
-        return lx.grad, lw.grad, None if lb is None else lb.grad
-
-    monkeypatch.setattr(zsi, "_scan_fwd", fake_scan_fwd)
-    monkeypatch.setattr(zsi, "_scan_bwd", fake_scan_bwd)
-    monkeypatch.setattr(zci, "_conv_fwd", fake_conv_fwd)
-    monkeypatch.setattr(zci, "_conv_bwd", fake_conv_bwd)
-    names = ["selective_scan_cuda", "causal_conv1d_cuda", "causal_conv1d", "causal_conv1d.causal_conv1d_interface", "_ref_ssi_under_shim"]
-    saved_mods = {n: sys.modules.get(n) for n in names}
+    g = gold("integration_shim")
+    saved_mods = {n: sys.modules.get(n) for n in gs.SHIM_MODULES}
     try:
-        exec(compile(shim, "INTEGRATION.md:zigma_shims.py", "exec"), {"__name__": "zigma_shims"})
-        assert "selective_scan_cuda" in sys.modules and "causal_conv1d_cuda" in sys.modules
-        # the reference's own Python on top of the shim modules (UNMODIFIED files, loaded by path)
-        _load("causal_conv1d", os.path.join(REF, "dis_causal_conv1d", "causal_conv1d", "__init__.py"))
-        ssi = _load("_ref_ssi_under_shim", os.path.join(REF, "dis_mamba", "mamba_ssm", "ops", "selective_scan_interface.py"))
-        conv = sys.modules["causal_conv1d"]
-
-        torch.manual_seed(0)
-        Bt, E, L, N = 2, 6, 24, 4
-        mk = lambda *s: torch.randn(*s, dtype=torch.float32)
-        base = dict(u=mk(Bt, E, L), delta=0.5 * torch.rand(Bt, E, L), A=-torch.rand(E, N) - 0.1, B=mk(Bt, N, L), C=mk(Bt, N, L), D=mk(E),
-                    z=mk(Bt, E, L), delta_bias=0.3 * mk(E))
-
-        def run(fn):
-            a = {k: v.clone().requires_grad_() for k, v in base.items()}
-            out, last = fn(a["u"], a["delta"], a["A"], a["B"], a["C"], a["D"], z=a["z"], delta_bias=a["delta_bias"], delta_softplus=True,
-                           return_last_state=True)
-            out.square().sum().backward()
-            return out, last, {k: v.grad for k, v in a.items()}
-        out, last, grads = run(ssi.selective_scan_fn)                 # reference autograd Function -> shim -> (fake) raw ops
-        ref_out, ref_last, ref_grads = run(ssi.selective_scan_ref)    # the reference's own pure-PyTorch oracle
-        assert torch.allclose(out, ref_out, rtol=1e-4, atol=1e-5) and torch.allclose(last, ref_last, rtol=1e-4, atol=1e-5)
-        for k in base:
-            assert torch.allclose(grads[k], ref_grads[k], rtol=1e-3, atol=1e-4), k
-        assert "scan_fwd" in calls and "scan_bwd" in calls
-
-        x, w, b = mk(Bt, E, L).requires_grad_(), mk(E, 4).requires_grad_(), mk(E).requires_grad_()
-        y = conv.causal_conv1d_fn(x, w, b, "silu")
-        y.sum().backward()
-        x2, w2, b2 = x.detach().clone().requires_grad_(), w.detach().clone().requires_grad_(), b.detach().clone().requires_grad_()
-        y2 = zo.causal_conv1d(x2, w2, b2, "silu")
-        y2.sum().backward()
-        assert torch.allclose(y, y2) and torch.allclose(x.grad, x2.grad, atol=1e-6) and torch.allclose(w.grad, w2.grad, atol=1e-5)
-        assert "conv_fwd" in calls and "conv_bwd" in calls
+        calls = gs.install_shim(monkeypatch.setattr)
+        fwd, bwd, conv_fwd, conv_bwd = _replay(g)
     finally:
         for n, m in saved_mods.items():
             if m is None:
                 sys.modules.pop(n, None)
             else:
                 sys.modules[n] = m
+    assert calls == ["scan_fwd", "scan_fwd", "scan_bwd", "conv_fwd", "conv_bwd"], calls
+    want = lambda k: torch.from_numpy(g["want_" + k])
+
+    # the reference reads `out, x, *rest = fwd(...)`, returns rest[0] (out_z) and x[:, :, -1, 1::2] as the last state
+    # (selective_scan_interface.py:37-47); `du, ddelta, dA, dB, dC, dD, ddelta_bias, *rest = bwd(...)` with dz = rest[0] and
+    # dB, dC squeezed back to the 3-D shape they came in (:62-68); against its own selective_scan_ref
+    assert len(fwd) == 3
+    assert torch.allclose(fwd[2], want("scan_out"), rtol=1e-4, atol=1e-5)
+    assert torch.allclose(fwd[1][:, :, -1, 1::2], want("scan_last"), rtol=1e-4, atol=1e-5)
+    du, ddelta, dA, dB, dC, dD, ddelta_bias, *rest = bwd
+    got = dict(u=du, delta=ddelta, A=dA, B=dB.squeeze(1), C=dC.squeeze(1), D=dD, z=rest[0], delta_bias=ddelta_bias)
+    for k in gs.SCAN_INPUTS:
+        assert torch.allclose(got[k], want("scan_grad_" + k), rtol=1e-3, atol=1e-4), k
+
+    # causal_conv1d_interface.py:20 returns the fwd result as is; :31 reads `dx, dweight, dbias = bwd(...)`; against causal_conv1d_ref
+    assert torch.allclose(conv_fwd[0], want("conv_y"), atol=1e-6)
+    assert len(conv_bwd) == 3
+    for k, v in zip(("x", "w", "b"), conv_bwd):
+        assert torch.allclose(v, want("conv_grad_" + k), atol=1e-5), k

@@ -34,14 +34,6 @@ def test_reference_golden_replay():
         assert np.allclose(a, b, rtol=1e-6, atol=1e-7, equal_nan=True), (k, np.nanmax(np.abs(a - b)))
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/transport"), reason="reference tree not present")
-def test_live_against_reference_transport():
-    ref = gg.run_all(gg.load_reference_transport())
-    got = gg.run_all(tp)
-    for k, v in ref.items():
-        assert np.allclose(got[k], v, rtol=1e-6, atol=1e-7, equal_nan=True), k
-
-
 def test_create_transport_eps_quirk_and_errors():
     tr = tp.create_transport("Linear", "noise")
     assert tr.train_eps == 1e-3 and tr.sample_eps is None      # transport/__init__.py:52-57 as written
